@@ -2,6 +2,7 @@
 """Headline benchmark: checkpoint GB/s and Snapshot.take() blocking ms (BASELINE.json), one process per GPU.
 
     python bench.py --gpus 1 --steps K --warmup W                       # this repo's engine, config C3
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR    # ... and write what the last timed step computed
     python bench.py --impl reference --gpus 1 --steps K --warmup W      # the UNMODIFIED reference (oracle/_ref)
     torchrun ... bench.py --gpus N ... [--config c2|c3|c4|c5]
 
@@ -21,10 +22,16 @@ T:benchmarks/ddp/main.py:62-70 (barrier + synchronize on both sides), max over r
   e2e_roofline      : the whole take against min(sum of the ranks' D2H link, host write sink), both measured in this
                       run with the engine's own ring and workers
   cpu_baseline      : the unmodified reference on a bounded sample (rank 0, N=1)
+
+--dump-outputs DIR writes, after the timed steps, the tensors in the snapshot of the last timed step (read back from
+its payload files; the restored table too for C5, whose headline is the restore) as DIR/<name>.npy, float32 or float64,
+so that two builds can be compared output for output: the inputs are seeded, and a snapshot larger than 64 MB is
+sampled at the same seeded element indices in every run.
 """
 from __future__ import annotations
 
 import argparse
+import io
 import json
 import os
 import shutil
@@ -33,9 +40,13 @@ import sys
 import tempfile
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is written into it
+
+import numpy as np  # noqa: E402
 
 import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
@@ -296,6 +307,84 @@ def dump_trace(ctx: Ctx, tag: str, traces, out_dir: str) -> dict:
     return summary
 
 
+# ---- --dump-outputs -------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def _tensor_pieces(snap_dir: str):
+    """(name, tensor entry) of every stored piece of every tensor in the snapshot's manifest, in manifest order."""
+    with open(os.path.join(snap_dir, ".snapshot_metadata")) as f:
+        manifest = json.load(f)["manifest"]
+    for path, e in manifest.items():
+        if e.get("type") == "Tensor":
+            pieces = [e]
+        elif e.get("type") == "ChunkedTensor":
+            pieces = [c["tensor"] for c in e["chunks"]]
+        elif e.get("type") in ("ShardedTensor", "DTensor"):
+            pieces = [s["tensor"] for s in e["shards"]]
+        else:
+            continue
+        for i, te in enumerate(pieces):
+            yield path.replace("/", ".") + (f".piece{i}" if len(pieces) > 1 else ""), te
+
+
+def _out_dtype(dtype: torch.dtype):
+    return np.float64 if dtype in (torch.float64, torch.int32, torch.int64) else np.float32
+
+
+def _sample(name: str, flat, numel: int, keep: int):
+    """All of flat (1-D, indexable) or `keep` of its elements at indices seeded by the name: the same in every run."""
+    if keep >= numel:
+        return flat[:numel]
+    idx = np.unique(np.random.default_rng(zlib.crc32(name.encode())).integers(0, numel, keep))
+    return flat[torch.from_numpy(idx).to(flat.device)] if isinstance(flat, torch.Tensor) else flat[idx]
+
+
+def _read_piece(snap_dir: str, te: dict, name: str, keep: int) -> np.ndarray:
+    dtype = getattr(torch, te["dtype"].split(".")[-1])
+    numel = 1
+    for d in te["shape"]:
+        numel *= d
+    path = os.path.join(snap_dir, te["location"])
+    lo = te["byte_range"][0] if te.get("byte_range") else 0
+    if te["serializer"] == "buffer_protocol":
+        esz = torch.empty(0, dtype=dtype).element_size()
+        raw = np.memmap(path, dtype={1: np.int8, 2: np.int16, 4: np.int32, 8: np.int64}[esz], mode="r", offset=lo, shape=(numel,))
+        vals = torch.from_numpy(np.array(_sample(name, raw, numel, keep))).view(dtype)
+    else:  # torch_save
+        with open(path, "rb") as f:
+            f.seek(lo)
+            blob = f.read(te["byte_range"][1] - lo) if te.get("byte_range") else f.read()
+        t = torch.load(io.BytesIO(blob), map_location="cpu", weights_only=True)
+        vals = _sample(name, t.reshape(-1), numel, keep)
+    return vals.to(torch.float64 if _out_dtype(dtype) is np.float64 else torch.float32).numpy()
+
+
+def dump_outputs(ctx: Ctx, snap_dir: str, extra=None) -> None:
+    """--dump-outputs: every tensor piece of the snapshot at snap_dir (+ `extra` {name: tensor}) as DIR/<name>.npy,
+    each sampled in proportion to its size when all of them would exceed DUMP_LIMIT_BYTES."""
+    out_dir = ctx.args.dump_outputs
+    if not out_dir or ctx.rank != 0:
+        return
+    items = [(n, te, 1) for n, te in _tensor_pieces(snap_dir)]
+    items += [(n, t, 0) for n, t in (extra or {}).items()]
+    sizes = []
+    for n, x, from_file in items:
+        dtype = getattr(torch, x["dtype"].split(".")[-1]) if from_file else x.dtype
+        numel = int(np.prod(x["shape"])) if from_file else x.numel()
+        sizes.append((numel, np.dtype(_out_dtype(dtype)).itemsize))
+    total = sum(n * b for n, b in sizes)
+    budget = DUMP_LIMIT_BYTES - 256 * len(items)  # .npy headers
+    os.makedirs(out_dir, exist_ok=True)
+    for (name, x, from_file), (numel, b) in zip(items, sizes):
+        keep = numel if total <= budget else max(1, numel * budget // total)
+        if from_file:
+            arr = _read_piece(snap_dir, x, name, keep)
+        else:
+            arr = _sample(name, x.detach().reshape(-1), numel, keep).to(torch.float64 if b == 8 else torch.float32).cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
+
+
 # ---- C3: FSDP-layout Llama-3-8B ---------------------------------------------------------------------------------
 C3_WORKLOAD = "C3: FSDP-layout Llama-3-8B bf16 sharded state_dict (291 tensors, 16.06 GB total, dim-0 sharded over n_gpus), Snapshot.take to local fs"
 
@@ -384,6 +473,7 @@ def run_c3(ctx: Ctx, T, impl_desc: str) -> None:
     ok = all(torch.equal(local[n][0], regen[n][0]) for n in local)
     del regen
     ok = bool(ctx.min(1.0 if ok else 0.0))
+    dump_outputs(ctx, ctx.path(keep_tag))
     ctx.cleanup(keep_tag)
 
     # -- async_take: how long the caller is blocked --
@@ -420,11 +510,11 @@ def run_c3(ctx: Ctx, T, impl_desc: str) -> None:
         "definition": "Snapshot.take(path, app_state) wall clock through the public API: planning collectives, device->host copies of this rank's payload, file writes, metadata commit; max over ranks.  value is this same quantity.",
     }
     line["steps_ms"] = [round(x, 2) for x in step_ms]
-    line["take_blocking_ms"] = {"async_take_returns_ms": mean(block_ms), "async_total_ms": mean(async_total_ms), "sync_take_ms": take_ms,
+    line["take_blocking_ms"] = {"async_take_returns_ms": mean(block_ms), "async_total_ms": mean(async_total_ms), "timed_async_takes": len(block_ms), "sync_take_ms": take_ms,
                                 "engine_device_done_ms": blocking_stats.get("device_done_ms"), "async_take_returns_ms_each": [round(x, 2) for x in block_ms],
                                 "phases_of_last_async_take_ms": {k: round(v, 2) for k, v in ((S.LAST_STATS.get("take_phases_ms") or {}) if ours else {}).items()},
                                 "write_phases_of_last_async_take_ms": {k: round(v, 2) for k, v in ((S.LAST_STATS.get("write_phases_ms") or {}) if ours else {}).items()}}
-    line["restore"] = {"value": payload_total / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s", "ms": mean(restore_ms), "verified_all_tensors_all_ranks": ok,
+    line["restore"] = {"value": payload_total / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s", "ms": mean(restore_ms), "timed_restores": len(restore_ms), "verified_all_tensors_all_ranks": ok,
                        "scatter_kernel_ms": load_stats.get("kernel_ms")}
     line["clocks"] = clocks
     host_cpu = cpu.report()
@@ -594,6 +684,7 @@ def run_c2(ctx: Ctx, T, impl_desc: str) -> None:
     # manifest facts
     man = T.Snapshot(ctx.path(keep)).get_manifest()
     n_entries = len(man)
+    dump_outputs(ctx, ctx.path(keep))
     ctx.cleanup(keep)
     take_ms = mean(step_ms)
     config = {"workload": "C2: DDP ResNet-50 (320 state_dict tensors) + Adam (exp_avg, exp_avg_sq, 0-d fp32 CPU step per parameter), replicated=['**'], partitioned write to local fs",
@@ -603,7 +694,7 @@ def run_c2(ctx: Ctx, T, impl_desc: str) -> None:
     line["e2e"] = {"value": line["value"], "unit": "GB/s", "ms_per_step": take_ms, "h2d_bytes_per_step": int(mean(st.get("table_h2d_bytes", 0) for st in per_step)) if ours else 0,
                    "d2h_bytes_per_step": int(payload // max(1, world)), "definition": "Snapshot.take wall clock, max over ranks; replicated payload counted once"}
     line["steps_ms"] = [round(x, 2) for x in step_ms]
-    line["restore"] = {"ms": mean(restore_ms), "value": payload * world / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s (every rank restores the full replicated state)", "verified": ok}
+    line["restore"] = {"ms": mean(restore_ms), "value": payload * world / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s (every rank restores the full replicated state)", "timed_restores": len(restore_ms), "verified": ok}
     line["manifest_entries"] = n_entries
     line["gpu_launches"] = int(launches)
     if ours:
@@ -691,6 +782,8 @@ def run_c4(ctx: Ctx, T, impl_desc: str) -> None:
         t3 = time.perf_counter()
         res.append({"blocked_ms": ctx.max((t1 - t0) * 1e3), "steps_ms_total": ctx.max((t2 - t1) * 1e3), "wait_after_steps_ms": ctx.max((t3 - t2) * 1e3),
                     "still_draining_after_steps": ctx.max(float(still))})
+        if k + 1 == a.steps:
+            dump_outputs(ctx, ctx.path(f"s{k}"))
         ctx.cleanup(f"s{k}")
     # a synchronous take for comparison: the loop is blocked for all of it
     sync_ms, _ = ctx.timed(lambda: T.Snapshot.take(ctx.path("sync"), app, **kw))
@@ -751,7 +844,7 @@ def run_c5(ctx: Ctx, T, impl_desc: str) -> None:
     # restore at half the world size on a sub-group; the other ranks idle
     half = max(1, world // 2)
     sub = dist.new_group(list(range(half))) if world > 1 else None
-    restore_ms, ok = [], True
+    restore_ms, ok, restored = [], True, {}
     if rank < half:
         split2 = -(-rows // half)
         lo2 = min(rank * split2, rows)
@@ -759,7 +852,7 @@ def run_c5(ctx: Ctx, T, impl_desc: str) -> None:
         t2 = torch.zeros(n2, cols, device=device)
         app2 = {"emb": T.StateDict(table=W.c5_sharded(t2, lo2, rows, cols, rank, device, process_group=sub))}
         snap = T.Snapshot(ctx.path(keep), pg=sub) if sub is not None else T.Snapshot(ctx.path(keep))
-        for rep in range(1 + min(a.steps, 3)):
+        for rep in range(1 + a.steps):  # one untimed warm-up restore, then --steps timed ones
             t2.zero_()
             if sub is not None:
                 dist.barrier(group=sub, device_ids=[device.index]) if dist.get_backend() == "nccl" else dist.barrier(group=sub)
@@ -773,15 +866,17 @@ def run_c5(ctx: Ctx, T, impl_desc: str) -> None:
         for b in range(0, n2, 1 << 20):
             m = min(1 << 20, n2 - b)
             ok = ok and bool(torch.equal(t2[b:b + m], W.c5_content(lo2 + b, m, cols, device)))
+        restored = {f"restored.{rank}.emb.table": t2}
     r_ms = ctx.max(mean(restore_ms) if restore_ms else 0.0)
     ok = bool(ctx.min(1.0 if ok else 0.0))
+    dump_outputs(ctx, ctx.path(keep), restored)
     ctx.cleanup(keep)
     s_ms = mean(save_ms)
     config = {"workload": f"C5: row-wise ShardedTensor {rows} x {cols} fp32 ({payload / 1e9:.1f} GB) saved at world_size {world}, restored at world_size {half} (reshard-on-load)",
               "world_size": world, "restore_world_size": half, "payload_bytes_total": int(payload), "target_fs": a.target_fs, "_dtype": "fp32 (byte copy)",
               "l2": "per-rank shards (>= 2 GB) exceed the 126 MB L2"}
     line = common_line(ctx, impl_desc, "reshard_restore_GBps", payload / 1e9 / (r_ms / 1e3), "GB/s", r_ms, config)
-    line["e2e"] = {"value": line["value"], "unit": "GB/s", "ms_per_step": r_ms, "h2d_bytes_per_step": int(payload // half), "d2h_bytes_per_step": 0,
+    line["e2e"] = {"value": line["value"], "unit": "GB/s", "ms_per_step": r_ms, "timed_restores": len(restore_ms), "h2d_bytes_per_step": int(payload // half), "d2h_bytes_per_step": 0,
                    "definition": "Snapshot.restore wall clock on the restoring ranks (file reads, host->device copies, scatter into the 2x larger local shard), max over ranks"}
     line["save"] = {"value": payload / 1e9 / (s_ms / 1e3), "unit": "GB/s", "ms": s_ms}
     line["verified_every_element_on_restoring_ranks"] = ok
@@ -824,6 +919,7 @@ def run_c1(ctx: Ctx, T, impl_desc: str) -> None:
         T.Snapshot(ctx.path(keep)).restore(app)
         restore_ms.append((time.perf_counter() - t0) * 1e3)
     ok = all(torch.equal(want[k], v) for k, v in model.state_dict().items())
+    dump_outputs(ctx, ctx.path(keep))
     ctx.cleanup(keep)
     ms = mean(take_ms)
     config = {"workload": f"C1: single-process Snapshot.take of a 1 GiB fp32 nn.Linear({n},{n}) state_dict held on the CPU to local fs (no GPU on the path)",
@@ -833,7 +929,7 @@ def run_c1(ctx: Ctx, T, impl_desc: str) -> None:
     line["n_gpus"] = 0
     line["e2e"] = {"value": line["value"], "unit": "GB/s", "ms_per_step": ms, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0, "definition": "Snapshot.take wall clock; host tensors, host engine"}
     line["steps_ms"] = [round(x, 1) for x in take_ms]
-    line["restore"] = {"value": payload / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s", "ms": mean(restore_ms), "verified": ok}
+    line["restore"] = {"value": payload / 1e9 / (mean(restore_ms) / 1e3), "unit": "GB/s", "ms": mean(restore_ms), "timed_restores": len(restore_ms), "verified": ok}
     line["host_cpu_during_take"] = cpu.report()
     line["gpu_launches"] = 0
     if a.impl == "reference":
@@ -882,7 +978,10 @@ def main() -> None:
     ap.add_argument("--c4-steps-during", type=int, default=8)
     ap.add_argument("--c5-rows", type=int, default=W.C5_ROWS)
     ap.add_argument("--cpu-dryrun", action="store_true", help="developer aid: run the code paths on CPU tensors with shrunken shapes (no GPU box needed); never a measurement")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write the tensors the last timed step computed as DIR/<name>.npy (<= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.cpu_dryrun and args.c5_rows == W.C5_ROWS:
         args.c5_rows = 100_000
 

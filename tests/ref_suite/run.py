@@ -1,9 +1,10 @@
-"""Runs the REFERENCE'S OWN test files against this package (build container only: needs /root/reference).
+"""Runs the REFERENCE'S OWN test files against this package (needs the copy of the reference that build() stages
+under oracle/_ref by oracle/make_ref.sh).
 
     python tests/ref_suite/run.py [test_file.py …] [pytest args…]
 
 A scratch directory gets a generated package ``torchsnapshot`` whose ``__path__`` is
-``[shims, <repo>/torchsnapshot_b200, /root/reference/torchsnapshot]``: ``torchsnapshot.batcher``,
+``[shims, <repo>/torchsnapshot_b200, <repo>/oracle/_ref/torchsnapshot]``: ``torchsnapshot.batcher``,
 ``.io_preparers.tensor``, ``.scheduler``, ``.snapshot`` … load OUR files (as a second, self-consistent copy of the
 package under the reference's name), while helper modules we do not mirror (``test_utils``, ``uvm_tensor`` …) load the
 reference's files, whose relative imports then bind to our modules.  Spawned worker processes (run_with_pet) import
@@ -16,8 +17,8 @@ import tempfile
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
 OURS = os.path.join(REPO, "torchsnapshot_b200")
-REF = "/root/reference/torchsnapshot"
-REF_TESTS = "/root/reference/tests"
+REF = os.path.join(REPO, "oracle", "_ref", "torchsnapshot")
+REF_TESTS = os.path.join(REPO, "oracle", "_ref", "tests")
 DEFAULT = [
     "test_flatten.py", "test_manifest.py", "test_chunked_tensor_io_preparer.py", "test_tensor_io_preparer.py", "test_batcher.py",
     "test_sharded_tensor_resharding.py", "test_sharded_tensor_io_preparer.py", "test_partitioner.py", "test_snapshot.py", "test_state_dict.py",
@@ -62,7 +63,7 @@ def make_overlay(work: str) -> None:
 
 if __name__ == "__main__":
     if not os.path.isdir(REF_TESTS):
-        print("reference tree not present; nothing to run")
+        print("oracle/_ref/tests not staged (oracle/make_ref.sh); nothing to run")
         sys.exit(0)
     import pytest
 

@@ -3,7 +3,7 @@ IPv4 getsockname(); SURVEY.md §4.  async_take is covered through this package's
 
 `torchsnapshot_b200.install()` puts the engine underneath the UNMODIFIED reference: its own
 Snapshot.take/restore keep producing the golden bytes, but the raw tensor traffic goes through
-libtsnap_b200.so.  Needs the reference tree (build container only)."""
+libtsnap_b200.so.  Needs the copy of the reference that build() stages under oracle/_ref (oracle/make_ref.sh)."""
 import os
 import sys
 
@@ -15,27 +15,24 @@ from tests.test_parity_cpu import _golden, assert_matches_golden
 from tests.util import snapshot_digest, wire_bytes
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-# the staged copy travels to the GPU box (oracle/make_ref.sh); the read-only tree only exists in the build container
-REF_PARENT = next((p for p in (os.path.join(ROOT, "oracle", "_ref"), "/root/reference") if os.path.isdir(os.path.join(p, "torchsnapshot"))), None)
-pytestmark = pytest.mark.skipif(REF_PARENT is None, reason="reference not staged (oracle/make_ref.sh) and /root/reference not present")
+# staged by build() (oracle/make_ref.sh); the staged copy travels with the working tree
+REF_PARENT = os.path.join(ROOT, "oracle", "_ref")
+pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF_PARENT, "torchsnapshot")), reason="reference not staged (oracle/make_ref.sh)")
 
 
 def test_staged_reference_is_the_unmodified_tree():
-    """oracle/_ref must be a verbatim copy: every file's sha256 equals the one recorded at staging time and, where the
-    read-only tree is present, the one of the file there."""
+    """oracle/_ref must be a verbatim copy: every file's sha256 equals the one oracle/make_ref.sh recorded from the
+    source tree at staging time, and no file was added."""
     import hashlib
 
-    staged = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.isdir(os.path.join(staged, "torchsnapshot")):
-        pytest.skip("not staged")
-    want = dict(reversed(ln.split(None, 1)) for ln in open(os.path.join(staged, "MANIFEST.sha256")).read().splitlines() if ln.strip())
+    staged = os.path.join(REF_PARENT, "torchsnapshot")
+    want = dict(reversed(ln.split(None, 1)) for ln in open(os.path.join(REF_PARENT, "MANIFEST.sha256")).read().splitlines() if ln.strip())
+    want = {rel.strip(): digest for rel, digest in want.items()}
     assert len(want) > 40
     for rel, digest in want.items():
-        rel = rel.strip()
-        assert hashlib.sha256(open(os.path.join(staged, "torchsnapshot", rel), "rb").read()).hexdigest() == digest, rel
-        src = os.path.join("/root/reference/torchsnapshot", rel)
-        if os.path.isdir("/root/reference/torchsnapshot"):
-            assert hashlib.sha256(open(src, "rb").read()).hexdigest() == digest, rel
+        assert hashlib.sha256(open(os.path.join(staged, rel), "rb").read()).hexdigest() == digest, rel
+    have = {"./" + os.path.relpath(os.path.join(dp, f), staged) for dp, _, fs in os.walk(staged) if "__pycache__" not in dp for f in fs}
+    assert have == set(want)
 
 
 @pytest.fixture()

@@ -1,5 +1,6 @@
 """N>1 path on CPU: two gloo ranks exercise replicated-state partitioning, per-rank state, sharded state,
-the manifest gather/consolidation, the store-based async commit and restore at a different world size."""
+the manifest gather/consolidation, the store-based async commit and restore at a different world size; the manifest
+is compared with the one the unmodified reference wrote for the same job (tests/golden/two_rank_replicated.json)."""
 import json
 import os
 import sys
@@ -12,7 +13,7 @@ import torch.multiprocessing as mp
 
 from tests.util import det_tensor, snapshot_digest, wire_bytes
 
-HAVE_REF = os.path.isdir("/root/reference/torchsnapshot")
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _rep_state():
@@ -36,15 +37,17 @@ def _build_state(rank: int, world: int):
     return rep, own, st, full
 
 
-def _worker(rank: int, world: int, store_path: str, root: str, use_ref: bool, mode: str):
+def _worker(rank: int, world: int, store_path: str, root: str, ref_parent, mode: str):
+    """ref_parent: None for this package, else the directory holding the reference's torchsnapshot package
+    (oracle/gen_golden.py)."""
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["LOCAL_WORLD_SIZE"] = str(world)  # as torchrun sets it: ranks share the host-wide pool of I/O tokens
     os.environ["TSNAP_B200_HOST_IO_TOKENS"] = "3"  # fewer tokens than workers: the semaphore path is exercised
     os.environ["TORCHSNAPSHOT_MAX_CHUNK_SIZE_BYTES_OVERRIDE"] = "8192"
     os.environ["TORCHSNAPSHOT_SLAB_SIZE_THRESHOLD_BYTES_OVERRIDE"] = "4096"
     dist.init_process_group("gloo", init_method=f"file://{store_path}", rank=rank, world_size=world)
-    if use_ref:
-        sys.path.insert(0, "/root/reference")
+    if ref_parent:
+        sys.path.insert(0, ref_parent)
         os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
         import torchsnapshot as M
     else:
@@ -74,9 +77,9 @@ def _worker(rank: int, world: int, store_path: str, root: str, use_ref: bool, mo
     dist.destroy_process_group()
 
 
-def _run(world, use_ref, mode, root):
+def _run(world, ref_parent, mode, root):
     store = tempfile.NamedTemporaryFile(delete=False)
-    mp.spawn(_worker, args=(world, store.name, root, use_ref, mode), nprocs=world, join=True)
+    mp.spawn(_worker, args=(world, store.name, root, ref_parent, mode), nprocs=world, join=True)
     if os.path.exists(store.name):
         os.unlink(store.name)
 
@@ -102,7 +105,7 @@ def _no_duplicate_locations(root):
 
 @pytest.mark.parametrize("mode", ["sync", "async"])
 def test_two_rank_take_restore(mode, tmp_path):
-    _run(2, False, mode, str(tmp_path))
+    _run(2, None, mode, str(tmp_path))
     meta = _no_duplicate_locations(str(tmp_path))
     assert meta["world_size"] == 2
     # replicated entries live under rank 0 only; the chunked one is stitched back together
@@ -127,33 +130,32 @@ def test_two_rank_take_restore(mode, tmp_path):
     assert snap.read_object("1/own/tag") == "rank1"
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
-def test_two_rank_manifest_equals_reference(tmp_path):
-    ours, theirs = tmp_path / "ours", tmp_path / "theirs"
-    ours.mkdir()
-    theirs.mkdir()
-    _run(2, False, "sync", str(ours))
-    _run(2, True, "sync", str(theirs))
-    a = snapshot_digest(str(ours / "snap"))
-    b = snapshot_digest(str(theirs / "snap"))
-    # chunk-level assignment of identical chunked tensors iterates a Python set (T:partitioner.py:119-124): the
-    # rank that writes each chunk of "big" is hash-order dependent in BOTH implementations, so compare everything
-    # except which slab those chunks landed in
-    def scrub(d):
-        m = json.loads(json.dumps(d["manifest"]))
-        for c in m["0/rep/big"]["chunks"]:
-            c["tensor"]["location"] = "*"
-            c["tensor"]["byte_range"] = None
-        return m
+def scrubbed_manifest(digest):
+    """The manifest without what is hash-order dependent: chunk-level assignment of identical chunked tensors iterates
+    a Python set (T:partitioner.py:119-124), so the rank that writes each chunk of "big" is hash-order dependent in
+    BOTH implementations; compare everything except which slab those chunks, and the slab members numbered after
+    them, landed in."""
+    m = json.loads(json.dumps(digest["manifest"]))
+    for c in m["0/rep/big"]["chunks"]:
+        c["tensor"]["location"] = "*"
+        c["tensor"]["byte_range"] = None
+    for e in m.values():
+        if e.get("type") == "Tensor" and str(e["location"]).startswith("batched/"):
+            e["location"], e["byte_range"] = "*", None
+    return m
 
-    assert a["manifest"].keys() == b["manifest"].keys()
-    sa, sb = scrub(a), scrub(b)
+
+def test_two_rank_manifest_equals_reference(tmp_path):
+    ours = tmp_path / "ours"
+    ours.mkdir()
+    _run(2, None, "sync", str(ours))
+    a = snapshot_digest(str(ours / "snap"))
+    theirs = json.load(open(os.path.join(GOLDEN, "two_rank_replicated.json")))
+    assert a["manifest"].keys() == theirs["manifest"].keys()
+    sa = scrubbed_manifest(a)
     for k in sa:
-        if sa[k].get("type") == "Tensor" and str(sa[k]["location"]).startswith("batched/"):
-            sa[k]["location"] = sb[k]["location"] = "*"  # slab numbering depends on the chunk placement above
-            sa[k]["byte_range"] = sb[k]["byte_range"] = None
-        assert sa[k] == sb[k], k
-    assert sum(v.get("nbytes", 0) for v in a["files"].values()) == sum(v.get("nbytes", 0) for v in b["files"].values())
+        assert sa[k] == theirs["manifest"][k], k
+    assert sum(v.get("nbytes", 0) for v in a["files"].values()) == theirs["payload_nbytes"]
 
 
 def _subgroup_worker(rank: int, world: int, store_path: str, root: str):

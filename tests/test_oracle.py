@@ -1,9 +1,8 @@
 """Pins the oracle (oracle/ref_port.py): golden fixtures made by the unmodified reference, the
-known-answer plans asserted by the reference's own tests, and — when /root/reference is present —
-the live reference on fresh inputs."""
+known-answer plans asserted by the reference's own tests, and the chunk plans the reference computed for
+random shapes (tests/golden/chunk_plans.json)."""
 import json
 import os
-import sys
 
 import pytest
 import torch
@@ -153,23 +152,14 @@ def test_ref_pipeline_round_trip_and_bytes(tmp_path):
         assert wire_bytes(tensors[k]) == wire_bytes(out[k]), k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/torchsnapshot"), reason="reference tree not present")
-def test_oracle_against_live_reference(tmp_path):
-    sys.path.insert(0, "/root/reference")
-    os.environ.setdefault("PYTHONDONTWRITEBYTECODE", "1")
-    try:
-        import torchsnapshot as ref
-        from torchsnapshot.io_preparers.chunked_tensor import ChunkedTensorIOPreparer
-        from torchsnapshot.io_preparers.sharded_tensor import ShardedTensorIOPreparer
-    finally:
-        sys.path.remove("/root/reference")
-    g = torch.Generator().manual_seed(1234)
-    for _ in range(25):
-        shape = [int(x) for x in torch.randint(1, 40, (int(torch.randint(1, 4, (1,), generator=g)),), generator=g)]
-        t = torch.zeros(shape, dtype=torch.float32)
-        limit = int(torch.randint(16, 4000, (1,), generator=g))
-        ref_plan = [(c.offsets, c.sizes) for c in ChunkedTensorIOPreparer.chunk_tensor(t, chunk_sz_bytes=limit)]
-        assert ref_plan == R.chunk_plan(shape, 4, limit)
-        dim = int(torch.randint(0, len(shape), (1,), generator=g))
-        ref_sub = ShardedTensorIOPreparer.subdivide_shard(t, [0] * len(shape), shape, dim, limit)
-        assert [(o, s) for _, o, s in ref_sub] == [(o, s) for _, o, s in R.subdivide_plan([0] * len(shape), shape, dim, 4, limit)]
+def test_oracle_against_live_reference():
+    """Against the reference's recorded output, not a live run of it: the chunk_tensor / subdivide_shard plans the
+    unmodified reference computed for 25 seeded random shapes and byte limits (tests/golden/chunk_plans.json, made by
+    oracle/gen_golden.py) equal the oracle's."""
+    gold = _golden("chunk_plans")
+    assert len(gold["cases"]) == 25
+    for c in gold["cases"]:
+        shape, limit, dim = c["shape"], c["limit"], c["dim"]
+        assert [[list(o), list(s)] for o, s in R.chunk_plan(shape, gold["elem_size"], limit)] == c["chunks"], c
+        got = R.subdivide_plan([0] * len(shape), shape, dim, gold["elem_size"], limit)
+        assert [[list(o), list(s)] for _, o, s in got] == c["subdivide"], c

@@ -1,9 +1,10 @@
 """Product path on CPU tensors (host engine, native file I/O) against the reference's golden outputs:
 the whole ``.snapshot_metadata`` (containers, primitives, tensor entries, slab byte ranges) and the
-sha256 of every raw payload file must be identical; plus interchangeability with the live reference
-when its tree is present."""
+sha256 of every raw payload file must be identical; plus restoring snapshots the reference wrote
+(tests/golden/ref_snapshots/)."""
 import json
 import os
+import shutil
 import sys
 import tempfile
 
@@ -16,7 +17,6 @@ from tests.cases import CASES, SHARDED_CASES, apply_knobs, build_sharded
 from tests.util import det_tensor, snapshot_digest, wire_bytes
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
-HAVE_REF = os.path.isdir("/root/reference/torchsnapshot")
 
 
 def _golden(name):
@@ -180,15 +180,12 @@ def test_failed_write_leaves_no_metadata(tmp_path):
     assert not (blocker / ".snapshot_metadata").exists()
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present")
 @pytest.mark.parametrize("name", ["dtypes_and_views", "chunked_slabbed", "model_adam"])
 def test_interchangeable_with_live_reference(name, tmp_path):
-    sys.path.insert(0, "/root/reference")
-    os.environ.setdefault("PYTHONDONTWRITEBYTECODE", "1")
-    try:
-        import torchsnapshot as ref
-    finally:
-        sys.path.remove("/root/reference")
+    """Against the reference's recorded output, not a live run of it: what this package writes is, file for file, the
+    snapshot the unmodified reference wrote for the same state (stored by oracle/gen_golden.py; torch_save pickles are
+    compared as present, not byte for byte), and this package restores the reference's snapshot.  The other direction
+    is test_reference_restores_what_this_package_wrote."""
     from torchsnapshot_b200.flatten import flatten
 
     build, knobs = CASES[name]
@@ -201,22 +198,53 @@ def test_interchangeable_with_live_reference(name, tmp_path):
                 v.zero_()
         return t
 
+    shutil.copytree(os.path.join(GOLDEN, "ref_snapshots", name), tmp_path / "theirs")
     with apply_knobs(knobs):
-        ours = B.Snapshot.take(str(tmp_path / "ours"), {"state": B.StateDict(**state)})
-        theirs = ref.Snapshot.take(str(tmp_path / "theirs"), {"state": ref.StateDict(**state)})
+        B.Snapshot.take(str(tmp_path / "ours"), {"state": B.StateDict(**state)})
         assert snapshot_digest(str(tmp_path / "ours")) == snapshot_digest(str(tmp_path / "theirs"))
-        # the reference reads what we wrote, we read what the reference wrote
-        t1 = ref.StateDict(**zeros())
-        ref.Snapshot(str(tmp_path / "ours")).restore({"state": t1})
+        # we read what the reference wrote
         t2 = B.StateDict(**zeros())
         B.Snapshot(str(tmp_path / "theirs")).restore({"state": t2})
     a = flatten(state, "x")[1]
-    for got in (flatten(dict(t1), "x")[1], flatten(dict(t2), "x")[1]):
-        for k in a:
-            if isinstance(a[k], torch.Tensor):
-                assert wire_bytes(a[k]) == wire_bytes(got[k]), k
-            else:
-                assert a[k] == got[k], k
+    got = flatten(dict(t2), "x")[1]
+    for k in a:
+        if isinstance(a[k], torch.Tensor):
+            assert wire_bytes(a[k]) == wire_bytes(got[k]), k
+        else:
+            assert a[k] == got[k], k
+
+
+REF_PARENT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
+
+
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF_PARENT, "torchsnapshot")), reason="reference not staged (oracle/make_ref.sh)")
+@pytest.mark.parametrize("name", ["dtypes_and_views", "chunked_slabbed", "model_adam"])
+def test_reference_restores_what_this_package_wrote(name, tmp_path):
+    """The unmodified reference (the copy build() stages under oracle/_ref) reads this package's snapshot."""
+    sys.path.insert(0, REF_PARENT)
+    os.environ.setdefault("PYTHONDONTWRITEBYTECODE", "1")
+    try:
+        import torchsnapshot as ref
+    finally:
+        sys.path.remove(REF_PARENT)
+    from torchsnapshot_b200.flatten import flatten
+
+    build, knobs = CASES[name]
+    state = build("cpu")
+    target = build("cpu")
+    for v in flatten(target, "x")[1].values():
+        if isinstance(v, torch.Tensor):
+            v.zero_()
+    with apply_knobs(knobs):
+        B.Snapshot.take(str(tmp_path / "ours"), {"state": B.StateDict(**state)})
+        t1 = ref.StateDict(**target)
+        ref.Snapshot(str(tmp_path / "ours")).restore({"state": t1})
+    a, got = flatten(state, "x")[1], flatten(dict(t1), "x")[1]
+    for k in a:
+        if isinstance(a[k], torch.Tensor):
+            assert wire_bytes(a[k]) == wire_bytes(got[k]), k
+        else:
+            assert a[k] == got[k], k
 
 
 def test_restore_detects_missing_and_truncated_payload(tmp_path):

@@ -1,6 +1,8 @@
-"""Round-2 GPU tests: parity at BASELINE scale against the oracle, the engine underneath the UNMODIFIED reference
-with CUDA tensors (install() + cross-restore both ways), arena-less / bounded-arena / nearly-full-HBM operation,
-O_DIRECT file I/O, restore ordering against the caller's stream, timeline + probes."""
+"""Round-2 GPU tests: parity at BASELINE scale against the oracle and against snapshots of the UNMODIFIED reference
+(tests/golden/, oracle/gen_golden.py), the engine underneath the unmodified reference with CUDA tensors (install() +
+cross-restore both ways), arena-less / bounded-arena / nearly-full-HBM operation, O_DIRECT file I/O, restore ordering
+against the caller's stream, timeline + probes."""
+import gzip
 import hashlib
 import json
 import os
@@ -22,6 +24,7 @@ from torchsnapshot_b200.flatten import flatten  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 DEV = "cuda:0"
 
 
@@ -52,7 +55,7 @@ def fresh_engines():
 @pytest.fixture()
 def ref():
     if not os.path.isdir(os.path.join(REF_DIR, "torchsnapshot")):
-        pytest.skip("oracle/_ref not staged (run oracle/make_ref.sh where /root/reference exists)")
+        pytest.skip("oracle/_ref not staged (oracle/make_ref.sh needs a checkout of the reference)")
     sys.path.insert(0, REF_DIR)
     try:
         import torchsnapshot
@@ -148,20 +151,24 @@ def test_c2_layout_matches_oracle(tmp_path, pg):
     assert st["n_tiles_lsu"] > 0, "unpadded slab members must exercise the LSU kernel"
 
 
-def test_c2_replicated_equals_unmodified_reference_on_cuda(ref, tmp_path, pg):
+def test_c2_replicated_equals_unmodified_reference_on_cuda(tmp_path, pg):
     """replicated=['**'] sends every request through the partitioner (which reorders them, T:partitioner.py:194-211)
-    before the batcher: compare with the UNMODIFIED reference run on the same CUDA app_state — manifests and every
-    payload file must be identical."""
+    before the batcher: compare with the UNMODIFIED reference run on the same CUDA app_state (its snapshot's digest,
+    tests/golden/c2_replicated_cuda.json.gz) — manifests and every payload file must be identical."""
     app_state, kw, payload = W.build_c2(B, 0, 1, torch.device(DEV), 0)
     B.Snapshot.take(str(tmp_path / "ours"), app_state, **kw)
-    ref.Snapshot.take(str(tmp_path / "ref"), app_state, **kw)
-    d_ours, d_ref = snapshot_digest(str(tmp_path / "ours")), snapshot_digest(str(tmp_path / "ref"))
+    d_ours = snapshot_digest(str(tmp_path / "ours"))
+    with gzip.open(os.path.join(GOLDEN, "c2_replicated_cuda.json.gz"), "rt") as f:
+        d_ref = json.load(f)
     assert d_ours["manifest"] == d_ref["manifest"]
     assert d_ours["files"] == d_ref["files"]
     assert sum(f["nbytes"] for f in d_ours["files"].values() if "nbytes" in f) == payload
 
 
 # ---- the engine underneath the unmodified reference, CUDA tensors --------------------------------------------------
+MIXED_KNOBS = {"slab": 1 << 16, "max_chunk": 1 << 20}
+
+
 def _mixed_cuda_state():
     return {
         # (an even element count: the reference truncates bf16 tensors with an odd count, DESIGN.md "divergences")
@@ -181,8 +188,7 @@ def test_install_under_unmodified_reference_with_cuda_tensors(ref, tmp_path, pg)
     from tests.cases import apply_knobs
 
     state = _mixed_cuda_state()
-    knobs = {"slab": 1 << 16, "max_chunk": 1 << 20}
-    with apply_knobs(knobs):
+    with apply_knobs(MIXED_KNOBS):
         # 1. the reference alone (its own pageable tensor.to('cpu') path)
         ref.Snapshot.take(str(tmp_path / "ref"), {"m": ref.StateDict(**state)})
         # 2. the reference with the engine installed underneath
@@ -211,6 +217,26 @@ def test_install_under_unmodified_reference_with_cuda_tensors(ref, tmp_path, pg)
         B.Snapshot(str(tmp_path / "ref")).restore({"m": t2})
         for k, v in state.items():
             assert wire_bytes(v) == wire_bytes(t1[k]) == wire_bytes(t2[k]), k
+
+
+def test_mixed_cuda_state_equals_unmodified_reference_snapshot(tmp_path, pg):
+    """This package's snapshot of the mixed CUDA state == the UNMODIFIED reference's snapshot of it (digest stored in
+    tests/golden/mixed_cuda.json), and it restores bit for bit."""
+    from tests.cases import apply_knobs
+
+    state = _mixed_cuda_state()
+    with open(os.path.join(GOLDEN, "mixed_cuda.json")) as f:
+        d_ref = json.load(f)
+    assert d_ref["knobs"] == MIXED_KNOBS
+    with apply_knobs(MIXED_KNOBS):
+        snap = B.Snapshot.take(str(tmp_path / "ours"), {"m": B.StateDict(**state)})
+        d_ours = snapshot_digest(str(tmp_path / "ours"))
+        assert d_ours["manifest"] == d_ref["manifest"]
+        assert d_ours["files"] == d_ref["files"]
+        tgt = B.StateDict(**{k: torch.zeros_like(v) for k, v in state.items()})
+        snap.restore({"m": tgt})
+    for k, v in state.items():
+        assert wire_bytes(v) == wire_bytes(tgt[k]), k
 
 
 # ---- HBM staging: arena-less, bounded, engine-owned, nearly full device ----------------------------------------------

@@ -190,10 +190,27 @@ def _raw_castable(src: torch.dtype, dst: torch.dtype) -> bool:
     return src in _FLOATS and dst in _FLOATS
 
 
+def _q_params_equal(a: torch.Tensor, b: torch.Tensor) -> bool:
+    if a.qscheme() != b.qscheme():
+        return False
+    if a.qscheme() == torch.per_tensor_affine:
+        return a.q_scale() == b.q_scale() and a.q_zero_point() == b.q_zero_point()
+    return (
+        a.q_per_channel_axis() == b.q_per_channel_axis()
+        and torch.equal(a.q_per_channel_scales(), b.q_per_channel_scales())
+        and torch.equal(a.q_per_channel_zero_points(), b.q_per_channel_zero_points())
+    )
+
+
 def tensor_copy(dst: torch.Tensor, src: torch.Tensor) -> None:
-    """``dst.copy_(src)`` with the reference's quantized-tensor caveat (T:io_preparers/tensor.py:385-409)."""
+    """``dst.copy_(src)`` with the reference's quantized-tensor caveat (T:io_preparers/tensor.py:385-409): a quantized
+    copy moves the storage and the qparams, so a view of a larger tensor (a chunk) whose qparams differ from the
+    source's gets the dequantized values instead; with equal qparams the integer values are copied as they are."""
     if src.is_quantized and (
-        not dst.is_quantized or dst.qscheme() != src.qscheme() or dst.dtype != src.dtype or dst._is_view()
+        not dst.is_quantized
+        or dst.qscheme() != src.qscheme()
+        or dst.dtype != src.dtype
+        or (dst._is_view() and not _q_params_equal(dst, src))
     ):
         src = src.dequantize()
     dst.detach().copy_(src)

@@ -2432,7 +2432,8 @@ int tsnap_host_execute(const tsnap_copy_desc* members, int32_t n, void* wire_buf
         for (int k = 0; k < nc.n; ++k) {
             const Member& m = nc.m[k];
             const uint64_t wire_off = (d.dst_space == TSNAP_SPACE_WIRE ? m.dst : m.src) - uint64_t(uintptr_t(wire_buf));
-            if (d.dst_space == TSNAP_SPACE_WIRE && wire_off + m.bytes > wire_nbytes)
+            const uint64_t trailer = (m.mode == kModeCast && (m.shift & 1)) ? 16 : 0;  // quantised: [scale][zero_point]
+            if (d.dst_space == TSNAP_SPACE_WIRE && wire_off + m.bytes + trailer > wire_nbytes)
                 return set_err(TSNAP_EINVAL, "member exceeds the wire buffer");
             // grains must not split a destination element of a cast
             const uint64_t g = grain / 16 * 16;

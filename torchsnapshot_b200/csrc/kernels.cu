@@ -650,12 +650,21 @@ __device__ __noinline__ void tile_transpose(const Member& m, uint32_t index, uns
 }
 
 // ---- fused cast -------------------------------------------------------------------------------
-__device__ __forceinline__ double load_elem(const char* p, uint32_t dt) {
+// raw element bits; a source that is not element aligned (a wire piece packed behind an odd-sized slab member) is
+// assembled byte by byte, little-endian: the mirror of store_bytes
+template <typename U>
+__device__ __forceinline__ U load_bits(const char* p, bool aligned) {
+    if (aligned) return *reinterpret_cast<const U*>(p);
+    U v = 0;
+    for (int i = 0; i < (int)sizeof(U); ++i) v |= (U)((U)(unsigned char)p[i] << (8 * i));
+    return v;
+}
+__device__ __forceinline__ double load_elem(const char* p, uint32_t dt, bool aligned) {
     switch (dt) {
-        case TSNAP_F16: return (double)__half2float(*reinterpret_cast<const __half*>(p));
-        case TSNAP_BF16: return (double)__bfloat162float(*reinterpret_cast<const __nv_bfloat16*>(p));
-        case TSNAP_F32: return (double)*reinterpret_cast<const float*>(p);
-        default: return *reinterpret_cast<const double*>(p);
+        case TSNAP_F16: return (double)__half2float(__ushort_as_half(load_bits<unsigned short>(p, aligned)));
+        case TSNAP_BF16: return (double)__bfloat162float(__ushort_as_bfloat16(load_bits<unsigned short>(p, aligned)));
+        case TSNAP_F32: return (double)__uint_as_float(load_bits<unsigned int>(p, aligned));
+        default: return __longlong_as_double((long long)load_bits<unsigned long long>(p, aligned));
     }
 }
 __device__ __forceinline__ void store_bytes(char* p, const void* v, int n, bool aligned) {
@@ -677,18 +686,18 @@ __device__ __forceinline__ uint8_t quantize_elem(float x, double scale, int64_t 
     return (uint8_t)(int8_t)q;
 }
 
-__device__ __forceinline__ void convert_store(char* p, uint32_t ddt, const char* sp, uint32_t sdt, bool aligned) {
-    // <=32-bit float sources convert through fp32 (exact widening), fp64 sources narrow directly:
-    // the same single rounding step torch's copy kernel performs.
+__device__ __forceinline__ void convert_store(char* p, uint32_t ddt, const char* sp, uint32_t sdt, bool aligned, bool src_aligned) {
+    // <=32-bit float sources convert through fp32 (exact widening).  fp64 sources narrow to fp32 directly and to
+    // fp16 / bf16 through fp32 (two roundings): torch's copy kernel has no direct double -> half conversion either.
     if (sdt == TSNAP_F64) {
-        const double x = *reinterpret_cast<const double*>(sp);
+        const double x = __longlong_as_double((long long)load_bits<unsigned long long>(sp, src_aligned));
         if (ddt == TSNAP_F32) { const float f = (float)x; store_bytes(p, &f, 4, aligned); }
-        else if (ddt == TSNAP_F16) { const __half h = __double2half(x); store_bytes(p, &h, 2, aligned); }
+        else if (ddt == TSNAP_F16) { const __half h = __float2half_rn((float)x); store_bytes(p, &h, 2, aligned); }
         else if (ddt == TSNAP_BF16) { const __nv_bfloat16 b = __float2bfloat16_rn((float)x); store_bytes(p, &b, 2, aligned); }
         else store_bytes(p, &x, 8, aligned);
         return;
     }
-    const float f = (float)load_elem(sp, sdt);
+    const float f = (float)load_elem(sp, sdt, src_aligned);
     if (ddt == TSNAP_F32) store_bytes(p, &f, 4, aligned);
     else if (ddt == TSNAP_F16) { const __half h = __float2half_rn(f); store_bytes(p, &h, 2, aligned); }
     else if (ddt == TSNAP_BF16) { const __nv_bfloat16 b = __float2bfloat16_rn(f); store_bytes(p, &b, 2, aligned); }
@@ -765,6 +774,9 @@ __device__ __noinline__ void tile_cast(const Member& m, uint32_t index) {
             e0 += n & ~uint64_t(7);  // the ragged tail (< 8 elements) goes through the scalar loop below
         }
     }
+    // the wire side of a load may sit at any byte offset (slab members are packed without padding)
+    bool src_aligned = (m.src % m.src_esz) == 0;
+    for (uint32_t i = 0; i < m.nouter; ++i) src_aligned = src_aligned && ((uint64_t)m.sstride[i] % m.src_esz) == 0;
     if (m.dst_dtype == TSNAP_QINT8 || m.dst_dtype == TSNAP_QUINT8) {
         // quantise-on-save: 1-byte destination elements, consecutive threads write consecutive bytes
         const bool is_signed = m.dst_dtype == TSNAP_QINT8;
@@ -772,7 +784,7 @@ __device__ __noinline__ void tile_cast(const Member& m, uint32_t index) {
             const uint64_t row = e / m.inner, col = e - row * m.inner;
             int64_t so, dofs;
             outer_offsets(m, row, &so, &dofs);
-            const float x = (float)load_elem(sb + so + col * m.src_esz, m.src_dtype);
+            const float x = (float)load_elem(sb + so + col * m.src_esz, m.src_dtype, src_aligned);
             reinterpret_cast<uint8_t*>(db + dofs)[col] = quantize_elem(x, m.q_scale, m.q_zero_point, is_signed);
         }
         if ((m.shift & 1) && hi == m.bytes && threadIdx.x < 16) {
@@ -788,7 +800,7 @@ __device__ __noinline__ void tile_cast(const Member& m, uint32_t index) {
         const uint64_t row = e / m.inner, col = e - row * m.inner;
         int64_t so, dofs;
         outer_offsets(m, row, &so, &dofs);
-        convert_store(db + dofs + col * m.dst_esz, m.dst_dtype, sb + so + col * m.src_esz, m.src_dtype, aligned);
+        convert_store(db + dofs + col * m.dst_esz, m.dst_dtype, sb + so + col * m.src_esz, m.src_dtype, aligned, src_aligned);
     }
 }
 

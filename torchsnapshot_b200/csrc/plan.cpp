@@ -129,7 +129,8 @@ int normalize_copy(const tsnap_copy_desc& d, uint64_t wire_base, bool allow_bulk
         } else {
             m.inner = 1;
         }
-        if (m.src % es) return fail(TSNAP_EINVAL, "cast source is not element aligned");
+        // the source may be element-misaligned (a wire piece behind an odd-sized slab member): tile_cast then
+        // assembles each element from bytes, host_copy_range reads through memcpy
     } else {
         if (nd > 0 && dims[nd - 1].ss == int64_t(es) && dims[nd - 1].ds == int64_t(ed)) {
             m.inner = uint64_t(dims[nd - 1].size) * ed;
@@ -254,22 +255,26 @@ static inline double load_as_double(const void* p, uint32_t dt) {
         default: { double x; std::memcpy(&x, p, 8); return x; }
     }
 }
-// torch's CPU quantize_val (non-FBGEMM build, c10::qint8/quint8): zero_point + nearbyint(value * (1.0f / scale))
+// torch's CPU quantisation (FBGEMM's scalar Quantize): zero_point + nearbyint(value * (1.0f / scale)) in float,
+// clamped in floating point before the conversion to an integer: a rounded value beyond the int64 range (inf, 1e30)
+// has no integer conversion and must saturate at the matching end of the range
 static inline uint8_t quantize_host(float x, double scale, int64_t zp, bool is_signed) {
     const float inv = 1.0f / float(scale);
-    int64_t q = zp + int64_t(std::nearbyint(x * inv));
-    const int64_t lo = is_signed ? -128 : 0, hi = is_signed ? 127 : 255;
-    q = q < lo ? lo : (q > hi ? hi : q);
-    return uint8_t(int8_t(q));
+    double q = double(zp) + double(std::nearbyint(x * inv));
+    const double lo = is_signed ? -128.0 : 0.0, hi = is_signed ? 127.0 : 255.0;
+    q = q > lo ? q : lo;  // also maps NaN to lo instead of an undefined conversion
+    q = q < hi ? q : hi;
+    return uint8_t(int8_t(int(q)));
 }
 
 static inline void store_from(void* p, uint32_t dt, const void* sp, uint32_t sdt) {
-    // convert through float when the source is <= 32 bit (exact), through double otherwise
+    // convert through float when the source is <= 32 bit (exact), through double otherwise.  torch has no direct
+    // double -> half conversion: an fp64 source reaches fp16 (and bf16) through fp32, rounded twice, and so does this
     if (sdt == TSNAP_F64) {
         double x;
         std::memcpy(&x, sp, 8);
         switch (dt) {
-            case TSNAP_F16: { _Float16 h = (_Float16)x; std::memcpy(p, &h, 2); break; }
+            case TSNAP_F16: { _Float16 h = (_Float16)float(x); std::memcpy(p, &h, 2); break; }
             case TSNAP_BF16: { uint16_t v = f32_to_bf16(float(x)); std::memcpy(p, &v, 2); break; }
             case TSNAP_F32: { float f = float(x); std::memcpy(p, &f, 4); break; }
             default: std::memcpy(p, &x, 8);
